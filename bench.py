@@ -351,6 +351,28 @@ def sweep_leg(fn, device, tol, batch, cells=None):
     return out
 
 
+# instances whose whole solution --dump-outputs writes: 64 x 0.6 MB (z, lam, mu, dt, pair duals of 4 vehicles in float64) = 39 MB
+DUMP_SAMPLE = 64
+
+
+def dump_outputs(out_dir, st, it, dbl, sol):
+    """What one step of the timed path returns, as float64 ``out_dir/<name>.npy``: the per-instance statistics of the whole batch
+    (status, iters, obj, cviol, dual_inf, compl_inf, elastic) and the solution of a fixed, seeded sample of instances (z, lam, mu,
+    dt, pair_lam, pair_mu, pair_s; ``instance`` holds their batch indices)."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    B = st.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_SAMPLE), replace=False))
+    sel = torch.as_tensor(idx, device=st.device)
+    arrays = {"status": st, "iters": it, **dict(zip(("obj", "cviol", "dual_inf", "compl_inf", "elastic"), dbl)), "instance": idx}
+    names = {"pl": "pair_lam", "pm": "pair_mu", "ps": "pair_s"}
+    arrays.update({names.get(k, k): v.index_select(0, sel) for k, v in sol.items()})
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if torch.is_tensor(a) else a
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -368,11 +390,17 @@ def main():
     ap.add_argument("--tight-batch", type=int, default=592)
     ap.add_argument("--sweep", action="store_true", help="add the scaling sweep (BASELINE.json configs[4]) at --sweep-batch instances per cell")
     ap.add_argument("--sweep-batch", type=int, default=1024)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy (float64; "
+                    "statistics of every instance, solutions of %d seeded instances) to compare two builds output for output" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs needs --impl ours in a single process")
     global_batch = args.batch * world if args.weak else args.batch
 
     from conflict_rez_b200.control.batch_planner import random_init_offsets, shard_instances
@@ -517,6 +545,9 @@ def main():
     t_dev = ev[0].elapsed_time(ev[1]) / 1e3
     # pipelined: the launches overlap, their individual durations include waiting for SMs -- the kernel time per step is the timed region / steps
     t_kernel = float(np.mean([a.elapsed_time(b) for a, b in ksolve_ms])) / 1e3 if ksolve_ms else t_dev / args.steps
+    if args.dump_outputs:  # the solution of the last step stays in the handle that ran it
+        last = pipe.solvers[(args.steps - 1) % len(pipe.solvers)] if pipe is not None else sv
+        dump_outputs(args.dump_outputs, st, it, dbl, last.fetch_solution())
     st_h, it_h = st.cpu().numpy(), it.cpu().numpy()
     converged = int((st_h >= 0).sum())
     sum_iters = float(it_h.sum())

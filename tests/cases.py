@@ -11,15 +11,16 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def load_golden(name):
-    d = np.load(os.path.join(GOLDEN, name + ".npz"))
+    d = dict(np.load(os.path.join(GOLDEN, name + ".npz")))
+    d.update(np.load(os.path.join(GOLDEN, name + "_multipliers.npz")))
     prob = CollocationProblem(
         n_sets=d["p_n_sets"], obs_A=d["p_obs_A"], obs_b=d["p_obs_b"], tube_A=d["p_tube_A"], tube_b=d["p_tube_b"], init_pose=d["p_init_pose"],
         final_heading=d["p_final_heading"], body_G=d["p_body_G"], body_g=d["p_body_g"], wb=float(d["p_wb"]), region=d["p_region"], limits=d["p_limits"],
         K=int(d["p_K"]), n_per_set=int(d["p_n_per_set"]), dmin=float(d["p_dmin"]), shrink_tube=float(d["p_shrink"]),
     )
-    has_pairs = "g_pl" in d.files
+    has_pairs = "g_pl" in d
     guess = CollocationGuess(d["g_z"], d["g_lam"], d["g_mu"], d["g_dt"], d["g_pl"] if has_pairs else None, d["g_pm"] if has_pairs else None, d["g_ps"] if has_pairs else None)
-    sol = {k[2:]: d[k] for k in d.files if k.startswith("s_")}
+    sol = {k[2:]: v for k, v in d.items() if k.startswith("s_")}
     return prob, guess, sol
 
 

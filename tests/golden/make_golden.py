@@ -34,10 +34,12 @@ def save(name, prob, guess, nlp, res):
     if guess.pair_lam is not None:
         out.update(g_pl=guess.pair_lam, g_pm=guess.pair_mu, g_ps=guess.pair_s)
     out.update(s_z=u["z"], s_dt=u["dt"], s_obj=res.obj, s_iters=res.iters, s_status=res.status, s_cviol=res.cviol, s_dual_inf=res.dual_inf)
-    # full primal-dual point in the oracle's own ordering (oracle/nlp.py): input of the KKT certificate of the unmodified
-    # reference NLP (oracle/reference_nlp.py)
-    out.update(s_lam=u["lam"], s_mu=u["mu"], s_pl=u["pair_lam"], s_pm=u["pair_mu"], s_ps=u["pair_s"], s_y=res.y, s_zL=res.zL, s_zU=res.zU)
+    out.update(s_lam=u["lam"], s_mu=u["mu"], s_pl=u["pair_lam"], s_pm=u["pair_mu"], s_ps=u["pair_s"])
     np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
+    # constraint and bound multipliers in the oracle's own ordering (oracle/nlp.py): with the above the full primal-dual point, input
+    # of the KKT certificate of the unmodified reference NLP (oracle/reference_nlp.py).  A file of their own keeps every fixture
+    # under 1 MB (the 4-vehicle instance is 1.3 MB in one file).
+    np.savez_compressed(os.path.join(HERE, name + "_multipliers.npz"), s_y=res.y, s_zL=res.zL, s_zU=res.zU)
     print(name, res.return_status, res.iters, res.obj, res.cviol)
 
 
