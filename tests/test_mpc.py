@@ -119,7 +119,8 @@ def test_mpc_residuals_step_and_solution_match_oracle(backend, mpc_case):
     yd[iy] = y
     sv.debug_set_iterate(0, y=yd)
     c_d, gl_d, f_d = sv.debug_eval(0)
-    dx_o, dy_o, c_o, gl_o = oracle_newton_step(nlp, x0, y, zLd[ix], zUd[ix], 0.1, 1e-3)
+    dx_o, dy_o, c_o, gl_o, res_o = oracle_newton_step(nlp, x0, y, zLd[ix], zUd[ix], 0.1, 1e-3)
+    assert max(res_o[1:]) <= 1e-10  # the reference step solves its system
     assert abs(f_d - nlp.f(x0)) <= 1e-11 * abs(f_d)
     assert np.abs(c_d[iy] - c_o).max() <= 1e-10 and np.abs(gl_d[ix] - gl_o).max() <= 1e-9 * np.abs(gl_o).max()
     dx_d, dy_d, ok = sv.debug_step(0, 0.1, 1e-3)
