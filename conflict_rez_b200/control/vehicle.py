@@ -21,7 +21,7 @@ from conflict_rez_b200.control.compute_sets import compute_initial_states, compu
 from conflict_rez_b200.obstacle_types import GeofenceRegion
 from conflict_rez_b200.problem import CollocationGuess, CollocationProblem
 from conflict_rez_b200.pytypes import VehiclePrediction, VehicleState
-from conflict_rez_b200.solver import RETURN_STATUS, ObcaSolver, SolveOptions
+from conflict_rez_b200.solver import HIST_FIELDS, HIST_STEP_FIELDS, RETURN_STATUS, ObcaSolver, SolveOptions
 from conflict_rez_b200.vehicle_types import VehicleBody, VehicleConfig
 
 
@@ -37,13 +37,28 @@ class ObcaSol:
         self.result, self.b, self._wall = result, b, wall
 
     def stats(self):
+        """``iterations`` is present when the solve recorded (``SolveOptions.history`` > 0): IPOPT's per-iteration record as a dict
+        of lists, one entry per iterate.  Its key names are those of CasADi's IPOPT plugin as recalled; they could not be checked
+        against an installed CasADi.  As in IPOPT's table, the step entries (d_norm, regularization_size, alpha_pr, alpha_du,
+        ls_trials) of entry k describe the step that produced iterate k, and entry 0 has zeros there."""
         r, b = self.result, self.b
-        return {
+        out = {
             "return_status": RETURN_STATUS.get(int(r.status[b]), "Unknown"),
             "iter_count": int(r.iters[b]),
             "t_wall_total": self._wall,
             "success": bool(r.status[b] >= 0),
         }
+        if r.history is not None:
+            rows = r.history[b, : min(int(r.history_count[b]), r.history.shape[1])]
+            step = np.zeros((len(rows), 5))  # reg, d_norm, alpha_pr, alpha_du, ls_trials of the step into each iterate
+            step[1:] = np.nan_to_num(rows[:-1, HIST_STEP_FIELDS], nan=0.0)
+            f = dict(zip(HIST_FIELDS, rows.T))
+            out["iterations"] = {
+                "obj": f["obj"].tolist(), "inf_pr": f["inf_pr"].tolist(), "inf_du": f["inf_du"].tolist(), "mu": f["mu"].tolist(),
+                "d_norm": step[:, 1].tolist(), "regularization_size": step[:, 0].tolist(), "alpha_pr": step[:, 2].tolist(),
+                "alpha_du": step[:, 3].tolist(), "ls_trials": step[:, 4].astype(int).tolist(),
+            }
+        return out
 
 
 class Vehicle(object):

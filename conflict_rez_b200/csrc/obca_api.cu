@@ -63,6 +63,9 @@ struct ObcaHandle {
   bool have_order;
   long long* d_prof;  // [slots][NPROF + 1]
   int64_t launches;
+  double* d_hist;       // iteration record [B][hist_cap][OBCA_HIST_FIELDS] (obca_set_history), nullptr: off
+  int32_t* d_hist_cnt;  // [B]
+  int hist_cap;
 };
 
 // Every entry point that touches the device runs on the handle's device and restores the caller's current device
@@ -239,7 +242,18 @@ struct SolveArgs {
   // debug modes: 0 = solve, 1 = eval at stored iterate, 2 = Newton step at stored iterate
   int mode, b_only;
   int rw_in_smem;  // Riccati work arena in dynamic shared memory (else per-slot global memory)
-  double dbg_mu, dbg_dw;
+  int hist_cap;
+  // The debug modes do not record and the solve has no debug arguments: the two share their slot, so that the iteration record
+  // leaves the kernel's parameter block (and the stack frame k_solve copies it to) at its size.
+  union {
+    struct {
+      double dbg_mu, dbg_dw;
+    };
+    struct {
+      double* hist;         // mode 0: iteration record [B][hist_cap][OBCA_HIST_FIELDS], NaN-filled before the launch; nullptr: off
+      int32_t* hist_count;  // mode 0: [B] heads evaluated per instance
+    };
+  };
 };
 
 OBCA_HDN void run_instance(const Ctx& ctx, const SolveArgs& A, const Lay& L, const Stat& S, int b, int slot, Shared* sh, double* RW) {
@@ -248,8 +262,13 @@ OBCA_HDN void run_instance(const Ctx& ctx, const SolveArgs& A, const Lay& L, con
   carve_work(W, L, A.work + (size_t)slot * A.wk_stride);
   W.ricg = A.rw_in_smem ? nullptr : A.rw + (size_t)slot * A.ric_stride;
   if (A.mode == 0) {
+    if (ctx.tid == 0) {  // read by the other threads only after the CTA barrier at the start of ipm_solve
+      sh->hist = A.hist ? A.hist + (size_t)b * A.hist_cap * OBCA_HIST_FIELDS : nullptr;
+      sh->hist_cap = A.hist_cap, sh->hist_n = 0, sh->hist_attempt = 0;
+    }
     if (L.mode == 0) ipm_solve<0>(ctx, L, S, A.o, A.cnt, A.xL, A.xU, A.bcls, W, RW, A.rw_stride, sh, A.res + b);
     else ipm_solve<1>(ctx, L, S, A.o, A.cnt, A.xL, A.xU, A.bcls, W, RW, A.rw_stride, sh, A.res + b);
+    if (ctx.tid == 0 && A.hist) A.hist_count[b] = sh->hist_n;
     return;
   }
   double f, gdt;
@@ -437,9 +456,17 @@ static void free_device(ObcaHandle* h) {
   h->d_iter = h->d_work = h->d_rw = nullptr, h->d_res = nullptr, h->d_counter = nullptr;
 }
 
+static void free_history(ObcaHandle* h) {
+  if (!h->d_hist) return;
+  dev_sync();  // a solve on another stream may still write the record: the frees are stream ordered on stream 0
+  dev_free(h->d_hist), dev_free(h->d_hist_cnt);
+  h->d_hist = nullptr, h->d_hist_cnt = nullptr, h->hist_cap = 0;
+}
+
 int obca_destroy(ObcaHandle* h) {
   if (!h) return 0;
   DeviceGuard guard(h->device);
+  free_history(h);
   free_device(h);
   delete h;
   return 0;
@@ -828,8 +855,10 @@ static SolveArgs make_args(ObcaHandle* h, int mode, int b) {
   A.res = h->d_res, A.B = h->dims.batch, A.counter = h->d_counter, A.mode = mode, A.b_only = b;
   A.order = h->have_order ? h->d_order : nullptr;
   A.prof = getenv("OBCA_PROFILE") ? h->d_prof : nullptr;
-  A.dbg_mu = 0, A.dbg_dw = 0;
   A.rw_in_smem = h->ric_stride == 0;
+  A.hist_cap = h->hist_cap;
+  if (mode == 0) A.hist = h->d_hist, A.hist_count = h->d_hist_cnt;
+  else A.dbg_mu = 0, A.dbg_dw = 0;  // the debug entry points do not record
   return A;
 }
 
@@ -841,6 +870,7 @@ static int launch(ObcaHandle* h, const SolveArgs& A, void* stream) {
   for (int k = 0; k < 8; ++k) sh.blo[k] = A.blo[k], sh.bhi[k] = A.bhi[k];
   double red[40];
   Ctx ctx{0, 1, red, nullptr, nullptr};
+  if (A.mode == 0 && A.hist) memset(A.hist, 0xFF, (size_t)A.B * A.hist_cap * OBCA_HIST_FIELDS * sizeof(double));  // all-ones bytes: a NaN
   if (A.mode != 0)
     run_instance(ctx, A, *A.L, *A.S, A.b_only, 0, &sh, A.rw);
   else
@@ -848,6 +878,8 @@ static int launch(ObcaHandle* h, const SolveArgs& A, void* stream) {
 #else
   cudaStream_t s = (cudaStream_t)stream;
   if (A.mode == 0) CUDA_OK(cudaMemsetAsync(h->d_counter, 0, sizeof(int), s));
+  // rows a solve does not reach read back as NaN (all-ones bytes), not as what the previous solve left there
+  if (A.mode == 0 && A.hist) CUDA_OK(cudaMemsetAsync(A.hist, 0xFF, (size_t)A.B * A.hist_cap * OBCA_HIST_FIELDS * sizeof(double), s));
   int grid = A.mode == 0 ? h->slots : 1;
   size_t smem = h->rw_stride * sizeof(double);
   if (smem) CUDA_OK(cudaFuncSetAttribute(k_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1013,6 +1045,37 @@ int obca_set_order(ObcaHandle* h, const int32_t* order_dev, void* stream) {
 int obca_solve(ObcaHandle* h, void* stream) {
   if (!h || !h->have_static) return fail("obca_solve: call obca_set_static first");
   return launch(h, make_args(h, 0, 0), stream);
+}
+
+int obca_set_history(ObcaHandle* h, int32_t capacity) {
+  if (!h) return fail("obca_set_history: null handle");
+  if (capacity < 0) return fail("obca_set_history: capacity must be >= 0");
+  DeviceGuard guard(h->device);
+  free_history(h);
+  if (capacity == 0) return 0;
+  const size_t B = (size_t)h->dims.batch;
+  if (dev_alloc((void**)&h->d_hist, B * capacity * OBCA_HIST_FIELDS * sizeof(double)) || dev_alloc((void**)&h->d_hist_cnt, B * sizeof(int32_t))) {
+    dev_free(h->d_hist);
+    h->d_hist = nullptr, h->d_hist_cnt = nullptr;
+    return fail("obca_set_history: device allocation failed");
+  }
+  h->hist_cap = capacity;
+  return 0;
+}
+
+int obca_get_history(ObcaHandle* h, double* rows, int32_t* count, void* stream) {
+  if (!h || !h->d_hist) return fail("obca_get_history: recording is off (call obca_set_history with a capacity > 0 before obca_solve)");
+  DeviceGuard guard(h->device);
+  const size_t B = (size_t)h->dims.batch, nrow = B * h->hist_cap * OBCA_HIST_FIELDS * sizeof(double);
+#ifdef OBCA_HOST_EMU
+  (void)stream;
+  if (rows) memcpy(rows, h->d_hist, nrow);
+  if (count) memcpy(count, h->d_hist_cnt, B * sizeof(int32_t));
+#else
+  if (rows) CUDA_OK(cudaMemcpyAsync(rows, h->d_hist, nrow, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  if (count) CUDA_OK(cudaMemcpyAsync(count, h->d_hist_cnt, B * sizeof(int32_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+#endif
+  return 0;
 }
 
 int obca_get_stats(ObcaHandle* h, int32_t* status, int32_t* iters, double* obj, double* cviol, double* dual_inf, double* compl_inf, double* elastic,

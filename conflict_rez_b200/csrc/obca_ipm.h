@@ -14,7 +14,35 @@ struct Shared {   // lives in shared memory on the device
   double filt_theta[FILTER_MAX], filt_phi[FILTER_MAX];
   unsigned long long bars[8];  // mbarriers of the staged flat passes
   double blo[8], bhi[8];       // bounds of the 8 bound classes (see BoundCls)
+  // iteration record (obca_set_history).  `hist` is set per instance before ipm_solve and read by every thread (it decides the
+  // extra reduction of d_norm); the rest is thread 0's bookkeeping, kept here rather than in registers of the hot loop
+  double* hist;          // rows of the current instance [hist_cap][OBCA_HIST_FIELDS], nullptr: not recording
+  int hist_cap, hist_n;  // capacity, heads evaluated so far
+  int hist_attempt;      // interior-point run of this instance (ipm_solve restarts)
+  int hist_trials, hist_flags;
+  double hist_dw, hist_dn;  // delta_w and max |dx| of the current step
 };
+
+// Row of the current head: fields 0..8 and 15, field 14 (flags) so far; the step fields stay NaN until hist_step.  Thread 0.
+OBCA_HD void hist_head(Shared* sh, int it, double f, double cviol, double theta, double dual_inf, double compl0, double mu, double E0,
+                       bool acceptable, double rho) {
+  const int k = sh->hist_n++;
+  sh->hist_flags = acceptable ? OBCA_HIST_F_ACCEPTABLE : 0, sh->hist_trials = 0;
+  if (k >= sh->hist_cap) return;
+  double* r = sh->hist + (size_t)k * OBCA_HIST_FIELDS;
+  r[OBCA_HIST_ITER] = it, r[OBCA_HIST_ATTEMPT] = sh->hist_attempt, r[OBCA_HIST_OBJ] = f, r[OBCA_HIST_INF_PR] = cviol, r[OBCA_HIST_THETA] = theta;
+  r[OBCA_HIST_INF_DU] = dual_inf, r[OBCA_HIST_COMPL] = compl0, r[OBCA_HIST_MU] = mu, r[OBCA_HIST_ERR] = E0;
+  r[OBCA_HIST_FLAGS] = sh->hist_flags, r[OBCA_HIST_RHO] = rho;
+}
+// Step fields of the current head's row, when its iteration ends (accepted step or barrier reset).  Thread 0.
+OBCA_HD void hist_step(Shared* sh, double alpha_pr, double alpha_du, int flags) {
+  const int k = sh->hist_n - 1;
+  if (k >= sh->hist_cap) return;
+  double* r = sh->hist + (size_t)k * OBCA_HIST_FIELDS;
+  r[OBCA_HIST_REG] = sh->hist_dw, r[OBCA_HIST_D_NORM] = sh->hist_dn, r[OBCA_HIST_ALPHA_PR] = alpha_pr, r[OBCA_HIST_ALPHA_DU] = alpha_du;
+  r[OBCA_HIST_LS_TRIALS] = sh->hist_trials;
+  r[OBCA_HIST_FLAGS] = sh->hist_flags | flags | (sh->hist_dw > 0 ? OBCA_HIST_F_INERTIA : 0);
+}
 
 // Simple bounds by class instead of two FP64 vectors: one byte per variable.  Class 0: free, 1: lower bound 0 (duals, slacks,
 // elastic variables), 2..7: the two-sided bounds of x, y, v, delta, a, w.  The flat passes stage the class bytes next to the
@@ -326,9 +354,7 @@ OBCA_HDN int ipm_attempt(const Ctx& ctx, const Lay& L, const Stat& S, const Opts
     double s_d = fmax(o.s_max, (s_y + s_z) / fmax(1.0, (double)(cnt.m_active + cnt.nb))) / o.s_max;
     double s_c = fmax(o.s_max, s_z / fmax(1.0, (double)cnt.nb)) / o.s_max;
     double E0 = fmax(fmax(dual_inf / s_d, cviol), compl0 / s_c);
-#ifdef OBCA_HOST_EMU
-    if (getenv("OBCA_TRACE")) printf("%4d f=%.8e th=%.2e du=%.2e co=%.2e mu=%.1e dw=%.1e\n", it, f, theta, dual_inf, compl0, mu, dw_last);
-#endif
+    if (ctx.tid == 0 && sh->hist) hist_head(sh, it, f, cviol, theta, dual_inf, compl0, mu, E0, E0 <= 1e-6 && cviol <= 1e-2 && compl0 <= 1e-2, S.rho);
     if (E0 <= o.tol && dual_inf <= o.dual_inf_tol && cviol <= o.constr_viol_tol && compl0 <= o.compl_inf_tol) {
       status = OBCA_SOLVE_SUCCEEDED;
       break;
@@ -368,6 +394,7 @@ OBCA_HDN int ipm_attempt(const Ctx& ctx, const Lay& L, const Stat& S, const Opts
         break;
     }
     force_mu = false;
+    if (ctx.tid == 0 && sh->hist && !sig_ready) sh->hist_flags |= OBCA_HIST_F_MU_LOWERED;  // sig_ready is cleared exactly when mu was lowered
     cta_sync(ctx);
     const double tau = fmax(o.tau_min, 1.0 - mu);
     // ---- gradient of the barrier Lagrangian, barrier objective and grad_phi'dx bookkeeping
@@ -420,13 +447,15 @@ OBCA_HDN int ipm_attempt(const Ctx& ctx, const Lay& L, const Stat& S, const Opts
       break;
     }
     if (dw > 0) dw_last = dw;
+    if (ctx.tid == 0 && sh->hist) sh->hist_dw = dw;
     // ---- dz, fraction to the boundary, directional derivative of the barrier objective
-    double a_pr = 1.0, a_du = 1.0, dphi = 0, rel = 0, r_pr = 0;
+    double a_pr = 1.0, a_du = 1.0, dphi = 0, rel = 0, r_pr = 0, dn = 0;
     {
       const double* const src[5] = {W.x, W.zL, W.zU, W.gphi, W.dx};
       flat_pass_b<5>(ctx, st, bc, src, L.nx, [&](int, const double* v, double lo, double hi) {
         const double xv = v[0], zl = v[1], zu = v[2], d = v[4];
         rel = fmax(rel, fabs(d) * rcp_pos(1.0 + fabs(xv)));
+        dn = fmax(dn, fabs(d));
         if (lo > -INFINITY) {
           const double ig = rcp_pos(xv - lo);
           const double dz = (mu - zl * d) * ig - zl;
@@ -458,6 +487,10 @@ OBCA_HDN int ipm_attempt(const Ctx& ctx, const Lay& L, const Stat& S, const Opts
     if (r_pr > tau) a_pr = tau / r_pr;
     a_du = cta_min(ctx, a_du);
     rel = cta_max(ctx, rel);
+    if (sh->hist) {  // the only reduction the record adds
+      dn = cta_max(ctx, dn);
+      if (ctx.tid == 0) sh->hist_dn = dn;
+    }
     dphi = cta_sum(ctx, dphi) - cta_sum(ctx, yJdx);
 #ifdef OBCA_HOST_EMU
     if (getenv("OBCA_TRACE")) {  // which variable limits the primal step
@@ -535,6 +568,7 @@ OBCA_HDN int ipm_attempt(const Ctx& ctx, const Lay& L, const Stat& S, const Opts
         sbar -= log(prod);
       }
       prof_mark(ctx, 24);
+      if (ctx.tid == 0 && sh->hist) ++sh->hist_trials;
       cta_sync(ctx);
       model_eval<MODE>(ctx, L, S, W, W.xt, nullptr, W.ct, nullptr, &ft, &gdt_t);
       double tht = 0;
@@ -575,14 +609,12 @@ OBCA_HDN int ipm_attempt(const Ctx& ctx, const Lay& L, const Stat& S, const Opts
       alpha *= 0.5;
     }
     cta_sync(ctx);
-#ifdef OBCA_HOST_EMU
-    if (getenv("OBCA_TRACE")) printf("       a_pr=%.3e a_du=%.3e alpha=%.3e a_min=%.3e dphi=%.3e dw=%.1e acc=%d\n", a_pr, a_du, alpha, a_min, dphi, dw, (int)accepted);
-#endif
     if (!accepted) {
       // IPOPT enters its feasibility-restoration phase here.  This solver has none; what it can do cheaply is leave the corner the
       // iterate is stuck in: raise the barrier parameter again (x10, at most mu_init), forget the filter and iterate on -- a larger mu
       // re-centres the slacks that blocked the step.  Three attempts, then Restoration_Failed as before.
       if (n_rescue < 3 && it < o.max_iter) {
+        if (ctx.tid == 0 && sh->hist) hist_step(sh, 0.0, 0.0, OBCA_HIST_F_RESET);  // no step taken
         ++n_rescue;
         mu = fmin(o.mu_init, 10.0 * mu);
         cta_sync(ctx);
@@ -596,6 +628,7 @@ OBCA_HDN int ipm_attempt(const Ctx& ctx, const Lay& L, const Stat& S, const Opts
       break;
     }
     // ---- accept the trial point (dz is recomputed from dx; x + alpha dx reproduces the trial point bit for bit)
+    if (ctx.tid == 0 && sh->hist) hist_step(sh, alpha, a_du, tiny_last ? OBCA_HIST_F_TINY_STEP : 0);
     const double iks = 1.0 / o.kappa_sigma;
     {
       const double* const src[4] = {W.x, W.zL, W.zU, W.dx};
@@ -753,6 +786,7 @@ OBCA_HDN void ipm_solve(const Ctx& ctx, const Lay& L, const Stat& S, const Opts&
       cta_sync(ctx);
     }
     ++restarts;
+    if (ctx.tid == 0) ++sh->hist_attempt;
   }
   cta_sync(ctx);
   // Which weight the next control step starts with: the l1 penalty is exact when it exceeds the multipliers of the hard distance rows

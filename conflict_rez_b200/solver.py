@@ -97,6 +97,8 @@ EXPORTS = [
     "obca_solve",
     "obca_get_solution",
     "obca_get_stats",
+    "obca_set_history",
+    "obca_get_history",
     "obca_launch_count",
     "obca_layout",
     "obca_debug_get_iterate",
@@ -144,6 +146,8 @@ def load_library(path: Optional[str] = None) -> ctypes.CDLL:
     lib.obca_solve.argtypes = [vp, vp]
     lib.obca_get_solution.argtypes = [vp] + [vp] * 7 + [vp]
     lib.obca_get_stats.argtypes = [vp] + [vp] * 7 + [vp]
+    lib.obca_set_history.argtypes = [vp, ctypes.c_int32]
+    lib.obca_get_history.argtypes = [vp, vp, vp, vp]
     lib.obca_launch_count.argtypes = [vp]
     lib.obca_launch_count.restype = ctypes.c_int64
     lib.obca_layout.argtypes = [vp, ctypes.POINTER(ctypes.c_int64), ctypes.c_int]
@@ -168,6 +172,15 @@ class SolveOptions:
     max_iter: int = 3000
     elastic_weight: float = 1e3
     refine_steps: int = -1  # iterative-refinement solves per Newton system; -1: none at tol > 1e-5, 2 at tight tolerances
+    history: int = 0  # rows of the iteration record kept per instance (BatchResult.history); 0: no record
+
+
+# Fields of one row of the iteration record, in the order of OBCA_HIST_ITER .. OBCA_HIST_RHO (include/obca.h).  Row r describes
+# iterate r and the step taken from it; rows without a step have NaN in reg .. ls_trials.
+HIST_FIELDS = ("iter", "attempt", "obj", "inf_pr", "theta", "inf_du", "compl", "mu", "err", "reg", "d_norm", "alpha_pr", "alpha_du", "ls_trials",
+               "flags", "rho")
+HIST_STEP_FIELDS = slice(9, 14)  # reg, d_norm, alpha_pr, alpha_du, ls_trials
+HIST_F_MU_LOWERED, HIST_F_INERTIA, HIST_F_TINY_STEP, HIST_F_RESET, HIST_F_ACCEPTABLE = 1, 2, 4, 8, 16
 
 
 @dataclass
@@ -186,9 +199,38 @@ class BatchResult:
     pair_lam: Optional[np.ndarray]
     pair_mu: Optional[np.ndarray]
     pair_s: Optional[np.ndarray]
+    history: Optional[np.ndarray] = None  # (B, capacity, len(HIST_FIELDS)) float64 iteration record, None when not recorded
+    history_count: Optional[np.ndarray] = None  # (B,) int32 heads evaluated per instance (may exceed the capacity)
 
     def return_status(self, b: int = 0) -> str:
         return RETURN_STATUS.get(int(self.status[b]), "Unknown")
+
+
+def format_history(result: BatchResult, b: int = 0) -> str:
+    """IPOPT's iteration table of instance ``b`` from its record.  As in IPOPT's output, the step columns of a line (``||d||``,
+    ``lg(rg)`` = log10 delta_w, ``alpha_du``, ``alpha_pr``, ``ls`` = line-search trials) describe the step that produced its iterate,
+    so line 0 has none.  The last column shows the flags: m = mu lowered and a = acceptable point at this iterate; i = inertia
+    correction, t = tiny step and r = barrier reset on the step that led to it."""
+    if result.history is None:
+        raise ValueError("format_history: the solve did not record (SolveOptions.history = 0)")
+    rows, n = result.history[b], int(result.history_count[b])
+    lines = ["iter att       objective   inf_pr   inf_du lg(mu)  ||d|| lg(rg) alpha_du alpha_pr   ls      rho flags"]
+    head_bits, step_bits = HIST_F_MU_LOWERED | HIST_F_ACCEPTABLE, HIST_F_INERTIA | HIST_F_TINY_STEP | HIST_F_RESET
+    prev = None
+    for r in rows[: min(n, rows.shape[0])]:
+        fl = int(r[14]) & head_bits
+        if prev is None or np.isnan(prev[11]):  # first line, or first line of a restarted attempt
+            step = "     -      -        -        -    -"
+        else:
+            fl |= int(prev[14]) & step_bits
+            rg = "%6.1f" % np.log10(prev[9]) if prev[9] > 0 else "     -"
+            step = "%6.1e %s %8.2e %8.2e %4d" % (prev[10], rg, prev[12], prev[11], int(prev[13]))
+        flags = "".join(c for c, bit in zip("mitra", (HIST_F_MU_LOWERED, HIST_F_INERTIA, HIST_F_TINY_STEP, HIST_F_RESET, HIST_F_ACCEPTABLE)) if fl & bit)
+        lines.append("%4d %3d %15.8e %8.2e %8.2e %6.2f %s %8.1e %s" % (int(r[0]), int(r[1]), r[2], r[3], r[5], np.log10(r[7]), step, r[15], flags))
+        prev = r
+    if n > rows.shape[0]:
+        lines.append("... %d more iterations past the capacity of %d rows" % (n - rows.shape[0], rows.shape[0]))
+    return "\n".join(lines)
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -298,6 +340,7 @@ class ObcaSolver:
         keep["colloc_A"], keep["colloc_B"] = np.ascontiguousarray(cA), np.ascontiguousarray(cB)
         st = ObcaStatic(wb=float(prob.wb), **{n: _np_ptr(a) for n, a in keep.items()})
         self._check(self.lib.obca_set_static(self.handle, ctypes.byref(st)))
+        self._set_history()
         self._stream = None
         self._staging = {}
 
@@ -359,6 +402,11 @@ class ObcaSolver:
         if getattr(self, "handle", None):
             self.lib.obca_destroy(self.handle)
             self.handle = None
+
+    def _set_history(self):
+        """Turn the iteration record on for ``self.opts.history`` rows per instance (obca_set_history)."""
+        if self.opts.history:  # a negative capacity is rejected by the library
+            self._check(self.lib.obca_set_history(self.handle, int(self.opts.history)))
 
     def __del__(self):
         try:
@@ -440,6 +488,16 @@ class ObcaSolver:
         self._check(self.lib.obca_get_stats(self.handle, _ptr(st), _ptr(it), *[_ptr(t) for t in dbl], self._stream_ptr()))
         return st, it, dbl
 
+    def fetch_history(self):
+        """Device copies of the iteration record of the last solve: rows (B, history, 16) float64 and counts (B,) int32, or
+        (None, None) when the solver does not record."""
+        if self.opts.history <= 0:
+            return None, None
+        rows = torch.empty((self.B, self.opts.history, len(HIST_FIELDS)), dtype=torch.float64, device=self.device)
+        cnt = torch.empty(self.B, dtype=torch.int32, device=self.device)
+        self._check(self.lib.obca_get_history(self.handle, _ptr(rows), _ptr(cnt), self._stream_ptr()))
+        return rows, cnt
+
     def fetch_solution(self):
         B, V, M, O, P = self.B, self.V, self.Mmax, self.O, self.P
         dev = self.device
@@ -466,10 +524,11 @@ class ObcaSolver:
         self.run()
         st, it, dbl = self.fetch_stats()
         sol = self.fetch_solution()
+        hist, hcnt = self.fetch_history()
         h = self._to_host([st, it, dbl[0], dbl[1], dbl[2], dbl[3], sol["z"], sol["lam"] if want_duals else None, sol["mu"] if want_duals else None,
-                           sol["dt"], sol.get("pl"), sol.get("pm"), sol.get("ps"), dbl[4]])
+                           sol["dt"], sol.get("pl"), sol.get("pm"), sol.get("ps"), dbl[4], hist, hcnt])
         return BatchResult(status=h[0], iters=h[1], obj=h[2], cviol=h[3], dual_inf=h[4], compl_inf=h[5], elastic=h[13], z=h[6], lam=h[7], mu=h[8], dt=h[9],
-                           pair_lam=h[10], pair_mu=h[11], pair_s=h[12])
+                           pair_lam=h[10], pair_mu=h[11], pair_s=h[12], history=h[14], history_count=h[15])
 
     # -- introspection for the parity tests --------------------------------------------------------------
     def layout(self):
@@ -664,6 +723,7 @@ class ObcaMpcSolver(ObcaSolver):
         keep = {n: np.ascontiguousarray(getattr(prob, n), dtype=np.float64) for n in ("obs_A", "obs_b", "body_G", "body_g", "region", "limits")}
         st = ObcaStatic(wb=float(prob.wb), mpc_dt=float(prob.dt), **{n: _np_ptr(a) for n, a in keep.items()})
         self._check(self.lib.obca_set_static(self.handle, ctypes.byref(st)))
+        self._set_history()
 
     def upload_params(self, cur, ref, others):
         B, N, P = self.B, self.Mmax, self.P
@@ -774,6 +834,7 @@ class ObcaStateWsSolver(ObcaMpcSolver):
         self._keep = keep
         st = ObcaStatic(wb=float(prob.wb), mpc_dt=float(prob.dt), **{n: _np_ptr(a) for n, a in keep.items()})
         self._check(self.lib.obca_set_static(self.handle, ctypes.byref(st)))
+        self._set_history()
 
     def solve_ws(self, init_state, z_guess) -> BatchResult:
         B, M = self.B, self.Mmax

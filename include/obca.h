@@ -165,6 +165,63 @@ int obca_get_solution(ObcaHandle* h, double* z, double* lam, double* mu, double*
 int obca_get_stats(ObcaHandle* h, int32_t* status, int32_t* iters, double* obj, double* cviol, double* dual_inf,
                    double* compl_inf, double* elastic, void* stream);
 
+/* ---- iteration record ---------------------------------------------------------------------------------------------------
+ * With recording on, obca_solve writes one row of OBCA_HIST_FIELDS doubles per head of the interior-point loop of every
+ * instance, i.e. per evaluation of the error measures and the convergence test -- IPOPT's iteration table.  Row r describes
+ * iterate r and the step taken from it (the convention of IPOPT's own table shifts the step columns down by one row; see
+ * solver.format_history).  Rows are stored instance-major (B, capacity, OBCA_HIST_FIELDS), independent of obca_set_order.
+ *
+ *   #  field      value
+ *   0  ITER       iteration counter at the head (it accumulates over the attempts of an instance)
+ *   1  ATTEMPT    0 for the first interior-point run of the instance, +1 per restart (dual restoration or raise of rho)
+ *   2  OBJ        objective f
+ *   3  INF_PR     max |c|
+ *   4  THETA      sum |c| (the filter's constraint-violation measure)
+ *   5  INF_DU     max |grad f + J'y - zL + zU|
+ *   6  COMPL      max complementarity gap * multiplier (at mu = 0)
+ *   7  MU         barrier parameter at the head, before this iteration's update
+ *   8  ERR        scaled overall error E_0 of the convergence test
+ *   9  REG        delta_w of the inertia correction used for the step (0: none)
+ *  10  D_NORM     max |dx|
+ *  11  ALPHA_PR   accepted primal step (0 when the line search failed)
+ *  12  ALPHA_DU   step of the bound multipliers (0 when the line search failed)
+ *  13  LS_TRIALS  trial points evaluated by the filter line search (0 for a tiny step)
+ *  14  FLAGS      OBCA_HIST_F_* bits
+ *  15  RHO        elastic penalty weight in force
+ *
+ * A row without a step (the last head of a solve, a failed step computation) has NaN in fields 9..13.  Rows past the capacity are
+ * not written but are counted; unwritten rows read back as NaN. */
+#define OBCA_HIST_FIELDS 16
+#define OBCA_HIST_ITER 0
+#define OBCA_HIST_ATTEMPT 1
+#define OBCA_HIST_OBJ 2
+#define OBCA_HIST_INF_PR 3
+#define OBCA_HIST_THETA 4
+#define OBCA_HIST_INF_DU 5
+#define OBCA_HIST_COMPL 6
+#define OBCA_HIST_MU 7
+#define OBCA_HIST_ERR 8
+#define OBCA_HIST_REG 9
+#define OBCA_HIST_D_NORM 10
+#define OBCA_HIST_ALPHA_PR 11
+#define OBCA_HIST_ALPHA_DU 12
+#define OBCA_HIST_LS_TRIALS 13
+#define OBCA_HIST_FLAGS 14
+#define OBCA_HIST_RHO 15
+#define OBCA_HIST_F_MU_LOWERED 1   /* mu was lowered at this head */
+#define OBCA_HIST_F_INERTIA 2      /* inertia correction: delta_w > 0 */
+#define OBCA_HIST_F_TINY_STEP 4    /* tiny-step rule: step accepted without line search */
+#define OBCA_HIST_F_RESET 8        /* line search failed, barrier parameter raised again (barrier reset) */
+#define OBCA_HIST_F_ACCEPTABLE 16  /* the iterate passed IPOPT's acceptable-point test */
+
+/* rows kept per instance for the following obca_solve calls; 0 (default) turns recording off.  Takes B * capacity *
+ * OBCA_HIST_FIELDS doubles of device memory from the stream-ordered pool, released by obca_destroy or a later call.
+ * The debug entry points (obca_debug_*) do not record. */
+int obca_set_history(ObcaHandle* h, int32_t capacity);
+/* the record of the last obca_solve: rows (B, capacity, OBCA_HIST_FIELDS) dev, may be NULL; count (B) dev int32 = heads
+ * evaluated (may exceed capacity), may be NULL.  An error when recording is off. */
+int obca_get_history(ObcaHandle* h, double* rows, int32_t* count, void* stream);
+
 /* number of kernels this handle has launched so far (bench.py "gpu_launches") */
 int64_t obca_launch_count(const ObcaHandle* h);
 
