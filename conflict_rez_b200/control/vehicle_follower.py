@@ -27,6 +27,11 @@ from conflict_rez_b200.vehicle_types import VehicleBody, VehicleConfig
 
 np.random.seed(0)  # vehicle_follower.py:29 (seeds the random initial obstacle duals of the first step)
 
+# Warm-start constants of the MPC loops (warm_start=True), from the sweep of tools/gpu_mpc_warm_start.py on the 4-vehicle scene
+# (profiles/r04_mpc_warm_start.json, DESIGN.md section 4): IPOPT's push of 1e-3 (pushes of 1e-6 / 1e-9 gave single steps of 97 - 572
+# iterations), and mu starting at 1e-5, next to the final mu of a tol 1e-2 solve.  They act only on warm-started solves.
+MPC_WARM_START_OPTIONS = dict(warm_start_bound_push=1e-3, warm_start_mult_bound_push=1e-3, warm_start_mu_init=1e-5)
+
 
 def simulate_plant(state: np.ndarray, u: np.ndarray, dt: float, wb: float, substeps: int = 100) -> np.ndarray:
     """[x, y, psi, v, delta] after dt under constant input [a, w] (the reference integrates the same ODE with IDAS)."""
@@ -200,13 +205,17 @@ class MultiDistributedFollower(object):
         self.single_results: Dict[str, VehiclePrediction] = {}
         self.final_results: Dict[str, VehiclePrediction] = {}
         self.solver = None
+        self.warm_start = False
 
-    def setup_multi_vehicles(self, dt: float = 0.1, N: int = 30, dmin: float = 0.05):
+    def setup_multi_vehicles(self, dt: float = 0.1, N: int = 30, dmin: float = 0.05, warm_start: bool = False):
+        """``warm_start``: from the second control step on, a vehicle whose previous solve succeeded starts from that solve's
+        primal-dual iterate shifted by one node (``ObcaSolver.shift_iterate`` / ``solve_warm``) instead of z = 1, y = 0, mu = 0.1."""
+        self.warm_start = warm_start
         for v in self.vehicles:
             v.plan_single_path(spline_ws=self.spline_ws_config[v.agent])
             v.get_others(self.vehicles)
         # one batched handle: instance b = vehicle b (same obstacles, body, horizon; n_others = V - 1)
-        self.solver = ObcaMpcSolver(self.vehicles[0].mpc_problem(dt, N, dmin, batch=len(self.vehicles)), SolveOptions(max_iter=600),
+        self.solver = ObcaMpcSolver(self.vehicles[0].mpc_problem(dt, N, dmin, batch=len(self.vehicles)), SolveOptions(max_iter=600, **MPC_WARM_START_OPTIONS),
                                     device=self.device, lib=self._lib)
         for v in self.vehicles:
             v.setup_controller(dt=dt, N=N, dmin=dmin, solver=self.solver)
@@ -214,6 +223,7 @@ class MultiDistributedFollower(object):
             self.single_results[v.agent] = v.reference_traj
 
     def solve(self, num_iter: int = 500):
+        sv, ok = self.solver, None
         for _ in range(num_iter):
             for v in self.vehicles:
                 v.get_others_pred(self.vehicles)  # Jacobi snapshot (vehicle_follower.py:636-637)
@@ -224,7 +234,16 @@ class MultiDistributedFollower(object):
             st = lambda k: np.stack([i[3][k] for i in inputs])
             guess = CollocationGuess(st("z")[:, None], st("lam")[:, None], st("mu")[:, None], np.zeros(len(inputs)), st("pl"), st("pm"), st("ps"))
             t0 = time.perf_counter()
-            res = self.solver.solve_step(cur, ref, others, guess)  # all vehicles of this control step in one launch
+            if self.warm_start and ok is not None:
+                # the stored iterates are last step's solutions: shift them, then write the guesses (the same user variables for the
+                # vehicles that succeeded, the shifted backup plan for the others), and start only the former warm
+                sv.set_params(sv.upload_params(cur, ref, others))
+                sv.shift_iterate()
+                sv.set_inputs(sv.upload(guess))
+                res = sv.solve_warm(ok.astype(np.int32))
+            else:
+                res = sv.solve_step(cur, ref, others, guess)  # all vehicles of this control step in one launch
+            ok = res.status >= 0
             dt_solve = time.perf_counter() - t0
             self.step_time.append(dt_solve)
             self.step_iters.append(int(np.max(res.iters)))
@@ -253,7 +272,10 @@ class DeviceMpcLoop(object):
     step in a CUDA graph and replays it.  Built from a ``MultiDistributedFollower`` after ``setup_multi_vehicles()`` so that both
     loops start from the same plans and the same (random) first-step duals; ``export()`` writes the state back."""
 
-    def __init__(self, mdf: "MultiDistributedFollower"):
+    def __init__(self, mdf: "MultiDistributedFollower", warm_start: bool = False):
+        """``warm_start``: from the second step on, every vehicle whose previous solve succeeded starts from that solve's primal-dual
+        iterate shifted by one node on the device (``obca_shift_iterate`` + ``obca_warm_start``), as in
+        ``MultiDistributedFollower.setup_multi_vehicles(warm_start=True)``; a vehicle that failed starts cold from its shifted plan."""
         import torch
 
         from conflict_rez_b200.solver import TrajectoryOps
@@ -295,6 +317,8 @@ class DeviceMpcLoop(object):
         self.steps_done = 0
         self.fail_count = torch.zeros(V, dtype=torch.int64, device=self.dev)
         self.iters_log, self.status_log, self.traj_log = [], [], []
+        self.warm_start = warm_start
+        self.prev_ok = None  # (V,) int32 status >= 0 of the last solve, once there was one (warm_start only)
 
     def _step(self, log=True):
         torch, sv, ops = self.torch, self.solver, self.ops
@@ -309,8 +333,13 @@ class DeviceMpcLoop(object):
             d["pl"] = ops.shift_horizon(self.pl.reshape(V * self.P, N, 4)).reshape(V, self.P, N, 4)
             d["pm"] = ops.shift_horizon(self.pm.reshape(V * self.P, N, 4)).reshape(V, self.P, N, 4)
             d["ps"] = ops.shift_horizon(self.ps.reshape(V * self.P, N, 2)).reshape(V, self.P, N, 2)
+        warm = self.warm_start and self.prev_ok is not None
+        if warm:
+            sv.shift_iterate()  # before set_inputs, which writes the same user variables for the vehicles that start warm
         sv.set_params({"cur": self.state, "ref": ref, "others": others})
         sv.set_inputs({k: v.contiguous() for k, v in d.items()})
+        if warm:
+            sv.arm_warm_start(self.prev_ok)
         sv.run()
         st, it, _ = sv.fetch_stats()
         sol = sv.fetch_solution()
@@ -324,6 +353,8 @@ class DeviceMpcLoop(object):
         self.state = ops.plant_step(self.state, self.pred_z[:, 0, 5:7].contiguous(), self.dt, self.wb)
         self.clock = self.clock + self.dt
         self.fail_count += (~ok).to(torch.int64)
+        if self.warm_start:
+            self.prev_ok = ok.to(torch.int32)
         if log:
             self.iters_log.append(it)
             self.status_log.append(st)
@@ -340,7 +371,7 @@ class DeviceMpcLoop(object):
                 self._step(log=False)
             torch.cuda.current_stream(self.dev).wait_stream(side)
             torch.cuda.synchronize(self.dev)
-            names = ("state", "clock", "pred_z", "pred_lam", "pred_mu", "pl", "pm", "ps")
+            names = ("state", "clock", "pred_z", "pred_lam", "pred_mu", "pl", "pm", "ps") + (("prev_ok",) if self.warm_start else ())
             static = {k: getattr(self, k).clone() for k in names}
             for k in names:
                 setattr(self, k, static[k])

@@ -66,6 +66,7 @@ struct ObcaHandle {
   double* d_hist;       // iteration record [B][hist_cap][OBCA_HIST_FIELDS] (obca_set_history), nullptr: off
   int32_t* d_hist_cnt;  // [B]
   int hist_cap;
+  double ws_bound_push, ws_mult_bound_push, ws_mu_init;  // ObcaOptions::warm_start_*, handed to the instances by obca_warm_start
 };
 
 // Every entry point that touches the device runs on the handle's device and restores the caller's current device
@@ -222,6 +223,51 @@ OBCA_HDN void pack_one(const Lay& L, double* iter, size_t it_stride, const PackA
       W.x[L.oDT] = A.dt[b];
   }
 }
+// stored iterate <-> user arrays x, zL, zU (B,nx), y (B,ny), and mu (B) from the results.  One "thread" per (instance, element
+// of x | zL | zU | y).
+struct IterArgs {
+  double* v[4];  // x, zL, zU, y
+  double* mu;    // get only
+};
+OBCA_HDN void iterate_item(const Lay& L, double* iter, size_t it_stride, const IterArgs& A, const Result* res, int b, int e, bool get) {
+  Scratch W;
+  carve_iterate(W, L, iter + (size_t)b * it_stride);
+  int k = e / L.nx;
+  if (k > 3) k = 3;
+  const int i = e - k * L.nx, n = k < 3 ? L.nx : L.ny;
+  double* in = (k == 0 ? W.x : k == 1 ? W.zL : k == 2 ? W.zU : W.y) + i;
+  if (A.v[k]) {
+    double* user = A.v[k] + (size_t)b * n + i;
+    if (get) *user = *in;
+    else *in = *user;
+  }
+  if (get && e == 0 && A.mu) A.mu[b] = res[b].mu;
+}
+static inline int iterate_elems(const Lay& L) { return 3 * L.nx + L.ny; }
+
+OBCA_HDN void warm_arm(Result& r, const int32_t* mask, const double* mu0, int b, double mu_init, double push, double mult_push) {
+  r.warm = mask ? mask[b] != 0 : 1;
+  r.mu0 = (mu0 && mu0[b] > 0) ? mu0[b] : mu_init;
+  r.ws_bound_push = push, r.ws_mult_bound_push = mult_push;
+}
+
+// MPC mode: one "thread" per (instance, node-minor row of x, zL, zU or y) moves the row one node towards the start, the last valid
+// node held.  Rows of x / zL / zU: every field before oDT (no tube slacks in MPC mode); rows of y: the dynamics rows YCOL (valid
+// nodes 0 .. N - 2, node N - 1 is padding and is not touched) and YOBS .. the end (YTUBE is empty).  YINIT, YCONT, YTERM are not
+// node-indexed.  A thread owns its row, so the shift is in place.
+OBCA_HDN void shift_iterate_row(const Lay& L, double* iter, size_t it_stride, int b, int r) {
+  Scratch W;
+  carve_iterate(W, L, iter + (size_t)b * it_stride);
+  const int N = L.Mv, xr = L.oDT / N, ycol = 5 * L.V;
+  double* row;
+  int nv = N;
+  if (r < 3 * xr) row = (r < xr ? W.x : r < 2 * xr ? W.zL : W.zU) + (size_t)(r % xr) * N;
+  else if (r < 3 * xr + ycol) row = W.y + L.oYCOL + (size_t)(r - 3 * xr) * N, nv = N - 1;
+  else row = W.y + L.oYOBS + (size_t)(r - 3 * xr - ycol) * N;
+  for (int n = 0; n + 1 < nv; ++n) row[n] = row[n + 1];
+}
+static inline int shift_rows(const Lay& L) { return 3 * (L.oDT / L.Mv) + 5 * L.V + (L.ny - L.oYOBS) / L.Mv; }
+
 static inline int pack_elems(const Lay& L) { return L.V * L.Mv * NZ + L.V * L.Mv * L.O * 4 + L.P * L.Mv * 4 + L.P * L.Mv * 2 + 1; }
 
 struct SolveArgs {
@@ -316,6 +362,19 @@ __global__ void k_pack(const Lay* L, double* iter, size_t it_stride, PackArgs A,
   if (g >= (size_t)B * ne) return;
   pack_one(*L, iter, it_stride, A, (int)(g / ne), (int)(g % ne), unpack);
 }
+__global__ void k_iterate(const Lay* L, double* iter, size_t it_stride, IterArgs A, const Result* res, int B, int ne, bool get) {
+  size_t g = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= (size_t)B * ne) return;
+  iterate_item(*L, iter, it_stride, A, res, (int)(g / ne), (int)(g % ne), get);
+}
+__global__ void k_shift_iterate(const Lay* L, double* iter, size_t it_stride, int B, int nr) {
+  int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g < B * nr) shift_iterate_row(*L, iter, it_stride, g / nr, g % nr);
+}
+__global__ void k_warm_arm(Result* res, int B, const int32_t* mask, const double* mu0, double mu_init, double push, double mult_push) {
+  int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b < B) warm_arm(res[b], mask, mu0, b, mu_init, push, mult_push);
+}
 __global__ void k_init_pose(const Lay* L, double* iter, size_t it_stride, const double* pose, int B) {
   int g = blockIdx.x * blockDim.x + threadIdx.x;
   int per = L->V * 3;
@@ -390,11 +449,13 @@ const char* obca_last_error(void) { return g_err.c_str(); }
 void obca_default_options(ObcaOptions* o) {
   o->tol = 1e-2, o->constr_viol_tol = 1e-2, o->dual_inf_tol = 1.0, o->compl_inf_tol = 1e-4;
   o->mu_init = 0.1, o->dmin = 0.05, o->shrink_tube = 0.5, o->elastic_weight = 1e3, o->max_iter = 3000, o->refine_steps = -1;
+  o->warm_start_bound_push = 1e-3, o->warm_start_mult_bound_push = 1e-3, o->warm_start_mu_init = 1e-3;
 }
 
 static void apply_options(ObcaHandle* h, const ObcaOptions* o) {
   h->opts.tol = o->tol, h->opts.constr_viol_tol = o->constr_viol_tol, h->opts.dual_inf_tol = o->dual_inf_tol;
   h->opts.compl_inf_tol = o->compl_inf_tol, h->opts.mu_init = o->mu_init, h->opts.max_iter = o->max_iter;
+  h->ws_bound_push = o->warm_start_bound_push, h->ws_mult_bound_push = o->warm_start_mult_bound_push, h->ws_mu_init = o->warm_start_mu_init;
   h->dmin = o->dmin, h->shrink = o->shrink_tube, h->rho = o->elastic_weight;
   h->opts.refine_steps = o->refine_steps >= 0 ? o->refine_steps : (o->tol > 1e-5 ? 0 : 2);
 }
@@ -1045,6 +1106,69 @@ int obca_set_order(ObcaHandle* h, const int32_t* order_dev, void* stream) {
 int obca_solve(ObcaHandle* h, void* stream) {
   if (!h || !h->have_static) return fail("obca_solve: call obca_set_static first");
   return launch(h, make_args(h, 0, 0), stream);
+}
+
+static int run_iterate(ObcaHandle* h, const IterArgs& A, bool get, void* stream) {
+  DeviceGuard guard(h->device);
+  const int B = h->dims.batch, ne = iterate_elems(h->L);
+#ifdef OBCA_HOST_EMU
+  (void)stream;
+  for (int b = 0; b < B; ++b)
+    for (int e = 0; e < ne; ++e) iterate_item(h->L, h->d_iter, h->it_stride, A, h->d_res, b, e, get);
+#else
+  const size_t tot = (size_t)B * ne;
+  k_iterate<<<(unsigned)((tot + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->d_L, h->d_iter, h->it_stride, A, h->d_res, B, ne, get);
+  h->launches++;
+  CUDA_OK(cudaGetLastError());
+#endif
+  return 0;
+}
+
+int obca_get_iterate(ObcaHandle* h, double* x, double* y, double* zL, double* zU, double* mu, void* stream) {
+  if (!h) return fail("obca_get_iterate: null handle");
+  if (!h->have_static) return fail("obca_get_iterate: call obca_set_static first");
+  IterArgs A = {{x, zL, zU, y}, mu};
+  return run_iterate(h, A, true, stream);
+}
+
+int obca_set_iterate(ObcaHandle* h, const double* x, const double* y, const double* zL, const double* zU, void* stream) {
+  if (!h) return fail("obca_set_iterate: null handle");
+  if (!h->have_static) return fail("obca_set_iterate: call obca_set_static first");
+  IterArgs A = {{const_cast<double*>(x), const_cast<double*>(zL), const_cast<double*>(zU), const_cast<double*>(y)}, nullptr};
+  return run_iterate(h, A, false, stream);
+}
+
+int obca_shift_iterate(ObcaHandle* h, void* stream) {
+  if (!h) return fail("obca_shift_iterate: null handle");
+  if (!h->have_static) return fail("obca_shift_iterate: call obca_set_static first");
+  if (h->L.mode != 1 || h->L.euler != 0) return fail("obca_shift_iterate: MPC mode only (not collocation or state warm start handles)");
+  DeviceGuard guard(h->device);
+  const int B = h->dims.batch, nr = shift_rows(h->L);
+#ifdef OBCA_HOST_EMU
+  (void)stream;
+  for (int g = 0; g < B * nr; ++g) shift_iterate_row(h->L, h->d_iter, h->it_stride, g / nr, g % nr);
+#else
+  k_shift_iterate<<<(B * nr + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->d_L, h->d_iter, h->it_stride, B, nr);
+  h->launches++;
+  CUDA_OK(cudaGetLastError());
+#endif
+  return 0;
+}
+
+int obca_warm_start(ObcaHandle* h, const int32_t* mask, const double* mu0, void* stream) {
+  if (!h) return fail("obca_warm_start: null handle");
+  if (!h->have_static) return fail("obca_warm_start: call obca_set_static first");
+  DeviceGuard guard(h->device);
+  const int B = h->dims.batch;
+#ifdef OBCA_HOST_EMU
+  (void)stream;
+  for (int b = 0; b < B; ++b) warm_arm(h->d_res[b], mask, mu0, b, h->ws_mu_init, h->ws_bound_push, h->ws_mult_bound_push);
+#else
+  k_warm_arm<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->d_res, B, mask, mu0, h->ws_mu_init, h->ws_bound_push, h->ws_mult_bound_push);
+  h->launches++;
+  CUDA_OK(cudaGetLastError());
+#endif
+  return 0;
 }
 
 int obca_set_history(ObcaHandle* h, int32_t capacity) {

@@ -370,6 +370,10 @@ struct Result {
   double elastic;  // largest elastic variable at the returned point
   int refines, restarts;  // correction solves of the refinement loop; dual restorations (obca_ipm.h)
   double rho_carry;       // MPC mode: raised penalty weight kept for the next control step of this vehicle (0: none)
+  // obca_warm_start: the next solve starts from the stored iterate (`warm`, cleared by that solve) with barrier parameter mu0 and the
+  // pushes of the warm_start_* options in force at the arm.  Here rather than in Opts: k_solve's parameter block keeps its size
+  int warm;
+  double mu0, ws_bound_push, ws_mult_bound_push;
 };
 
 // ------------------------------------------------------------------------------------------------

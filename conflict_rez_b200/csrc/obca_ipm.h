@@ -21,13 +21,16 @@ struct Shared {   // lives in shared memory on the device
   int hist_attempt;      // interior-point run of this instance (ipm_solve restarts)
   int hist_trials, hist_flags;
   double hist_dw, hist_dn;  // delta_w and max |dx| of the current step
+  int hist_warm;            // the next head is the first of a warm-started attempt
+  int warm;                 // Result::warm of the current instance, set by thread 0 in ipm_solve, cleared after the first attempt
 };
 
 // Row of the current head: fields 0..8 and 15, field 14 (flags) so far; the step fields stay NaN until hist_step.  Thread 0.
 OBCA_HD void hist_head(Shared* sh, int it, double f, double cviol, double theta, double dual_inf, double compl0, double mu, double E0,
                        bool acceptable, double rho) {
   const int k = sh->hist_n++;
-  sh->hist_flags = acceptable ? OBCA_HIST_F_ACCEPTABLE : 0, sh->hist_trials = 0;
+  sh->hist_flags = (acceptable ? OBCA_HIST_F_ACCEPTABLE : 0) | (sh->hist_warm ? OBCA_HIST_F_WARM : 0), sh->hist_trials = 0;
+  sh->hist_warm = 0;
   if (k >= sh->hist_cap) return;
   double* r = sh->hist + (size_t)k * OBCA_HIST_FIELDS;
   r[OBCA_HIST_ITER] = it, r[OBCA_HIST_ATTEMPT] = sh->hist_attempt, r[OBCA_HIST_OBJ] = f, r[OBCA_HIST_INF_PR] = cviol, r[OBCA_HIST_THETA] = theta;
@@ -250,7 +253,8 @@ OBCA_HDN void push_into_bounds(const Ctx& ctx, const Lay& L, const double* xL, c
   cta_sync(ctx);
 }
 
-// One interior-point run from the point in W.x (slack initialisation, push into the bounds, z = 1, y = 0, mu = mu_init).
+// One interior-point run from the point in W.x (slack initialisation, push into the bounds, z = 1, y = 0, mu = mu_init; with
+// sh->warm from the stored zL, zU, y and mu0, see obca_warm_start in obca.h).
 // `it` and `n_refine` accumulate over the runs of one instance.  Returns the status; *el_out = largest elastic variable.
 template <int MODE>
 OBCA_HDN int ipm_attempt(const Ctx& ctx, const Lay& L, const Stat& S, const Opts& o, const Counts& cnt, const double* xL,
@@ -260,25 +264,30 @@ OBCA_HDN int ipm_attempt(const Ctx& ctx, const Lay& L, const Stat& S, const Opts
   assume_scratch(W);
   OBCA_ASSUME_STATIC(L, S);
   OBCA_ASSUME_GLOBAL(xL), OBCA_ASSUME_GLOBAL(xU);
-  // ---- initial point
+  // ---- initial point.  Warm start (IPOPT warm_start_init_point): the stored x, zL, zU, y of the instance instead of z = 1, y = 0
   init_slacks<MODE>(ctx, L, S, W);
-  push_into_bounds(ctx, L, xL, xU, W.x, o.bound_push, o.bound_frac);
+  const bool warm = sh->warm;  // after the barrier that ends init_slacks (ipm_solve clears it before a restart)
+  push_into_bounds(ctx, L, xL, xU, W.x, warm ? res->ws_bound_push : o.bound_push, warm ? res->ws_bound_push : o.bound_frac);
   for (int q = ctx.tid; q < L.nx; q += ctx.nt) {
-    W.zL[q] = xL[q] > -INFINITY ? 1.0 : 0.0;
-    W.zU[q] = xU[q] < INFINITY ? 1.0 : 0.0;
+    const double zl0 = warm ? fmax(W.zL[q], res->ws_mult_bound_push) : 1.0, zu0 = warm ? fmax(W.zU[q], res->ws_mult_bound_push) : 1.0;
+    W.zL[q] = xL[q] > -INFINITY ? zl0 : 0.0;
+    W.zU[q] = xU[q] < INFINITY ? zu0 : 0.0;
     W.dx[q] = 0, W.dzL[q] = 0, W.dzU[q] = 0, W.gl[q] = 0;
   }
-  for (int q = ctx.tid; q < L.ny; q += ctx.nt) W.y[q] = 0, W.dy[q] = 0;
-  if (ctx.tid == 0) sh->filt_n = 0;
+  for (int q = ctx.tid; q < L.ny; q += ctx.nt) {
+    if (!warm) W.y[q] = 0;
+    W.dy[q] = 0;
+  }
+  if (ctx.tid == 0) sh->filt_n = 0, sh->hist_warm = warm;
   cta_sync(ctx);
-  double mu = o.mu_init;
+  const double mu_min = fmin(o.tol, o.compl_inf_tol) / (o.kappa_eps + 1.0);
+  double mu = warm ? fmax(mu_min, res->mu0) : o.mu_init;
   double f, gdt;
   model_eval<MODE>(ctx, L, S, W, W.x, W.y, W.c, W.gl, &f, &gdt);
   double th0 = 0;
   for (int q = ctx.tid; q < L.ny; q += ctx.nt) th0 += fabs(W.c[q]);
   th0 = cta_sum(ctx, th0);
   const double theta_max = 1e4 * fmax(1.0, th0), theta_min = 1e-4 * fmax(1.0, th0);
-  const double mu_min = fmin(o.tol, o.compl_inf_tol) / (o.kappa_eps + 1.0);
   double dw_last = 0.0;
   bool tiny_last = false, force_mu = false;
   // IPOPT acceptable-point bookkeeping: acceptable_tol 1e-6, acceptable_iter 15
@@ -755,6 +764,10 @@ OBCA_HDN void ipm_solve(const Ctx& ctx, const Lay& L, const Stat& S, const Opts&
   // MPC mode: the solves of one handle are consecutive control steps of the same vehicle; a weight that had to be raised stays
   // raised for the next step (the geometry that made the penalty inexact is still there) and is dropped after a failed solve
   const double carry = MODE == 1 ? res->rho_carry : 0.0;
+  if (ctx.tid == 0) {  // the arm of obca_warm_start is consumed by this solve
+    sh->warm = res->warm;
+    res->warm = 0;
+  }
   cta_sync(ctx);
   if (carry > rho0) {
     if (ctx.tid == 0) *rho = carry;
@@ -786,7 +799,7 @@ OBCA_HDN void ipm_solve(const Ctx& ctx, const Lay& L, const Stat& S, const Opts&
       cta_sync(ctx);
     }
     ++restarts;
-    if (ctx.tid == 0) ++sh->hist_attempt;
+    if (ctx.tid == 0) ++sh->hist_attempt, sh->warm = 0;  // restarts start cold (read after the barriers of init_slacks)
   }
   cta_sync(ctx);
   // Which weight the next control step starts with: the l1 penalty is exact when it exceeds the multipliers of the hard distance rows

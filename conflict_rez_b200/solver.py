@@ -59,6 +59,9 @@ class ObcaOptions(ctypes.Structure):
         ("elastic_weight", ctypes.c_double),
         ("max_iter", ctypes.c_int32),
         ("refine_steps", ctypes.c_int32),
+        ("warm_start_bound_push", ctypes.c_double),
+        ("warm_start_mult_bound_push", ctypes.c_double),
+        ("warm_start_mu_init", ctypes.c_double),
     ]
 
 
@@ -99,6 +102,10 @@ EXPORTS = [
     "obca_get_stats",
     "obca_set_history",
     "obca_get_history",
+    "obca_get_iterate",
+    "obca_set_iterate",
+    "obca_shift_iterate",
+    "obca_warm_start",
     "obca_launch_count",
     "obca_layout",
     "obca_debug_get_iterate",
@@ -108,6 +115,11 @@ EXPORTS = [
     "obca_debug_kkt_apply",
     "obca_debug_profile",
 ]
+
+
+# SolveOptions fields that go to the library's ObcaOptions under the same name
+_C_OPTIONS = ("tol", "constr_viol_tol", "dual_inf_tol", "compl_inf_tol", "mu_init", "max_iter", "elastic_weight", "refine_steps",
+              "warm_start_bound_push", "warm_start_mult_bound_push", "warm_start_mu_init")
 
 
 def default_library_path() -> str:
@@ -148,6 +160,10 @@ def load_library(path: Optional[str] = None) -> ctypes.CDLL:
     lib.obca_get_stats.argtypes = [vp] + [vp] * 7 + [vp]
     lib.obca_set_history.argtypes = [vp, ctypes.c_int32]
     lib.obca_get_history.argtypes = [vp, vp, vp, vp]
+    lib.obca_get_iterate.argtypes = [vp] + [vp] * 5 + [vp]
+    lib.obca_set_iterate.argtypes = [vp] + [vp] * 4 + [vp]
+    lib.obca_shift_iterate.argtypes = [vp, vp]
+    lib.obca_warm_start.argtypes = [vp, vp, vp, vp]
     lib.obca_launch_count.argtypes = [vp]
     lib.obca_launch_count.restype = ctypes.c_int64
     lib.obca_layout.argtypes = [vp, ctypes.POINTER(ctypes.c_int64), ctypes.c_int]
@@ -173,6 +189,10 @@ class SolveOptions:
     elastic_weight: float = 1e3
     refine_steps: int = -1  # iterative-refinement solves per Newton system; -1: none at tol > 1e-5, 2 at tight tolerances
     history: int = 0  # rows of the iteration record kept per instance (BatchResult.history); 0: no record
+    # warm start from the stored iterate (ObcaSolver.arm_warm_start / solve_warm), IPOPT's options of the same names
+    warm_start_bound_push: float = 1e-3
+    warm_start_mult_bound_push: float = 1e-3
+    warm_start_mu_init: float = 1e-3
 
 
 # Fields of one row of the iteration record, in the order of OBCA_HIST_ITER .. OBCA_HIST_RHO (include/obca.h).  Row r describes
@@ -180,7 +200,7 @@ class SolveOptions:
 HIST_FIELDS = ("iter", "attempt", "obj", "inf_pr", "theta", "inf_du", "compl", "mu", "err", "reg", "d_norm", "alpha_pr", "alpha_du", "ls_trials",
                "flags", "rho")
 HIST_STEP_FIELDS = slice(9, 14)  # reg, d_norm, alpha_pr, alpha_du, ls_trials
-HIST_F_MU_LOWERED, HIST_F_INERTIA, HIST_F_TINY_STEP, HIST_F_RESET, HIST_F_ACCEPTABLE = 1, 2, 4, 8, 16
+HIST_F_MU_LOWERED, HIST_F_INERTIA, HIST_F_TINY_STEP, HIST_F_RESET, HIST_F_ACCEPTABLE, HIST_F_WARM = 1, 2, 4, 8, 16, 32
 
 
 @dataclass
@@ -209,13 +229,13 @@ class BatchResult:
 def format_history(result: BatchResult, b: int = 0) -> str:
     """IPOPT's iteration table of instance ``b`` from its record.  As in IPOPT's output, the step columns of a line (``||d||``,
     ``lg(rg)`` = log10 delta_w, ``alpha_du``, ``alpha_pr``, ``ls`` = line-search trials) describe the step that produced its iterate,
-    so line 0 has none.  The last column shows the flags: m = mu lowered and a = acceptable point at this iterate; i = inertia
-    correction, t = tiny step and r = barrier reset on the step that led to it."""
+    so line 0 has none.  The last column shows the flags: m = mu lowered, a = acceptable point and w = warm-started attempt at this
+    iterate; i = inertia correction, t = tiny step and r = barrier reset on the step that led to it."""
     if result.history is None:
         raise ValueError("format_history: the solve did not record (SolveOptions.history = 0)")
     rows, n = result.history[b], int(result.history_count[b])
     lines = ["iter att       objective   inf_pr   inf_du lg(mu)  ||d|| lg(rg) alpha_du alpha_pr   ls      rho flags"]
-    head_bits, step_bits = HIST_F_MU_LOWERED | HIST_F_ACCEPTABLE, HIST_F_INERTIA | HIST_F_TINY_STEP | HIST_F_RESET
+    head_bits, step_bits = HIST_F_MU_LOWERED | HIST_F_ACCEPTABLE | HIST_F_WARM, HIST_F_INERTIA | HIST_F_TINY_STEP | HIST_F_RESET
     prev = None
     for r in rows[: min(n, rows.shape[0])]:
         fl = int(r[14]) & head_bits
@@ -225,7 +245,7 @@ def format_history(result: BatchResult, b: int = 0) -> str:
             fl |= int(prev[14]) & step_bits
             rg = "%6.1f" % np.log10(prev[9]) if prev[9] > 0 else "     -"
             step = "%6.1e %s %8.2e %8.2e %4d" % (prev[10], rg, prev[12], prev[11], int(prev[13]))
-        flags = "".join(c for c, bit in zip("mitra", (HIST_F_MU_LOWERED, HIST_F_INERTIA, HIST_F_TINY_STEP, HIST_F_RESET, HIST_F_ACCEPTABLE)) if fl & bit)
+        flags = "".join(c for c, bit in zip("mitraw", (HIST_F_MU_LOWERED, HIST_F_INERTIA, HIST_F_TINY_STEP, HIST_F_RESET, HIST_F_ACCEPTABLE, HIST_F_WARM)) if fl & bit)
         lines.append("%4d %3d %15.8e %8.2e %8.2e %6.2f %s %8.1e %s" % (int(r[0]), int(r[1]), r[2], r[3], r[5], np.log10(r[7]), step, r[15], flags))
         prev = r
     if n > rows.shape[0]:
@@ -327,7 +347,7 @@ class ObcaSolver:
             dims.n_sets[a] = int(prob.n_sets[a])
         copts = ObcaOptions()
         self.lib.obca_default_options(ctypes.byref(copts))
-        for name in ("tol", "constr_viol_tol", "dual_inf_tol", "compl_inf_tol", "mu_init", "max_iter", "elastic_weight", "refine_steps"):
+        for name in _C_OPTIONS:
             setattr(copts, name, getattr(self.opts, name))
         copts.dmin, copts.shrink_tube = prob.dmin, prob.shrink_tube
         self.handle = ctypes.c_void_p()
@@ -521,6 +541,52 @@ class ObcaSolver:
         """Host arrays in, host arrays out: H2D copies, batched solve, D2H copies."""
         d = self.upload(guess, init_pose)
         self.set_inputs(d)
+        return self._run_and_fetch(want_duals)
+
+    def solve_warm(self, mask=None, mu0=None, want_duals: bool = True) -> BatchResult:
+        """Solve again from the stored iterates (the last solve's, or ``put_iterate`` / ``shift_iterate``) without uploading a guess:
+        ``arm_warm_start(mask, mu0)``, batched solve, D2H copies.  Unarmed instances start cold from the stored x."""
+        self.arm_warm_start(mask, mu0)
+        return self._run_and_fetch(want_duals)
+
+    # -- warm start from the stored primal-dual iterate (obca_get_iterate ... obca_warm_start) ----------------------------------------
+    def fetch_iterate(self):
+        """Device copies of the stored iterate of every instance in the internal layout (``layout()``): x, zL, zU (B,nx), y (B,ny)
+        and mu (B), the barrier parameter at the end of the last solve."""
+        L = self.layout()
+        dev, B = self.device, self.B
+        d = {k: torch.empty((B, L["nx"]), dtype=torch.float64, device=dev) for k in ("x", "zL", "zU")}
+        d["y"] = torch.empty((B, L["ny"]), dtype=torch.float64, device=dev)
+        d["mu"] = torch.empty(B, dtype=torch.float64, device=dev)
+        self._check(self.lib.obca_get_iterate(self.handle, _ptr(d["x"]), _ptr(d["y"]), _ptr(d["zL"]), _ptr(d["zU"]), _ptr(d["mu"]), self._stream_ptr()))
+        return d
+
+    def put_iterate(self, d):
+        """Write x, zL, zU, y (device tensors shaped as ``fetch_iterate`` returns them; a missing key keeps that part) into the stored
+        iterate; ``mu`` is not stored (pass it to ``arm_warm_start``)."""
+        L = self.layout()
+        shapes = {"x": L["nx"], "zL": L["nx"], "zU": L["nx"], "y": L["ny"]}
+        t = {}
+        for k, n in shapes.items():
+            if d.get(k) is not None:
+                t[k] = torch.as_tensor(d[k], dtype=torch.float64, device=self.device).contiguous()
+                if tuple(t[k].shape) != (self.B, n):
+                    raise ValueError("put_iterate: %s must have shape (%d, %d), got %s" % (k, self.B, n, tuple(t[k].shape)))
+        self._check(self.lib.obca_set_iterate(self.handle, _ptr(t.get("x")), _ptr(t.get("y")), _ptr(t.get("zL")), _ptr(t.get("zU")), self._stream_ptr()))
+
+    def shift_iterate(self):
+        """MPC mode: move the stored iterate of every instance one node ahead, last node held (``_adv_onestep`` of the whole
+        primal-dual point)."""
+        self._check(self.lib.obca_shift_iterate(self.handle, self._stream_ptr()))
+
+    def arm_warm_start(self, mask=None, mu0=None):
+        """The next solve starts instance b from its stored iterate when ``mask[b]`` is true (None: every instance), with barrier
+        parameter ``mu0[b]`` (None: ``warm_start_mu_init``).  The solve consumes the arm."""
+        self._arm = [None if a is None else torch.as_tensor(a, dtype=dt, device=self.device).reshape(self.B).contiguous()
+                     for a, dt in ((mask, torch.int32), (mu0, torch.float64))]  # alive until the kernel has read them
+        self._check(self.lib.obca_warm_start(self.handle, _ptr(self._arm[0]), _ptr(self._arm[1]), self._stream_ptr()))
+
+    def _run_and_fetch(self, want_duals: bool) -> BatchResult:
         self.run()
         st, it, dbl = self.fetch_stats()
         sol = self.fetch_solution()
@@ -714,7 +780,7 @@ class ObcaMpcSolver(ObcaSolver):
         dims = ObcaDims(batch=self.B, V=1, O=self.O, K=5, n_per_set=1, mode=1, horizon=prob.N, n_others=prob.n_others)
         copts = ObcaOptions()
         self.lib.obca_default_options(ctypes.byref(copts))
-        for name in ("tol", "constr_viol_tol", "dual_inf_tol", "compl_inf_tol", "mu_init", "max_iter", "elastic_weight", "refine_steps"):
+        for name in _C_OPTIONS:
             setattr(copts, name, getattr(self.opts, name))
         copts.dmin = prob.dmin
         self.handle = ctypes.c_void_p()
@@ -818,7 +884,7 @@ class ObcaStateWsSolver(ObcaMpcSolver):
         dims.n_sets[0] = prob.n_sets
         copts = ObcaOptions()
         self.lib.obca_default_options(ctypes.byref(copts))
-        for name in ("tol", "constr_viol_tol", "dual_inf_tol", "compl_inf_tol", "mu_init", "max_iter", "elastic_weight", "refine_steps"):
+        for name in _C_OPTIONS:
             setattr(copts, name, getattr(self.opts, name))
         copts.shrink_tube = float(prob.shrink_tube)
         self.handle = ctypes.c_void_p()

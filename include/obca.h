@@ -72,6 +72,10 @@ typedef struct ObcaOptions {
   int32_t max_iter;
   int32_t refine_steps;          /* iterative-refinement solves per Newton system (IPOPT: max_refinement_steps); -1 = automatic:
                                     0 when tol > 1e-5 (the reference's 1e-2), 2 at tight tolerances */
+  /* warm start (obca_warm_start), IPOPT's options of the same names; defaults 1e-3, 1e-3, 1e-3 */
+  double warm_start_bound_push;      /* bound_push and bound_frac of the push of the stored x into its bounds */
+  double warm_start_mult_bound_push; /* floor of the stored bound multipliers */
+  double warm_start_mu_init;         /* barrier parameter of a warm start without its own mu0 */
 } ObcaOptions;
 
 typedef struct ObcaStatic {       /* host pointers; copied by obca_set_static */
@@ -213,6 +217,7 @@ int obca_get_stats(ObcaHandle* h, int32_t* status, int32_t* iters, double* obj, 
 #define OBCA_HIST_F_TINY_STEP 4    /* tiny-step rule: step accepted without line search */
 #define OBCA_HIST_F_RESET 8        /* line search failed, barrier parameter raised again (barrier reset) */
 #define OBCA_HIST_F_ACCEPTABLE 16  /* the iterate passed IPOPT's acceptable-point test */
+#define OBCA_HIST_F_WARM 32        /* first head of an attempt that started from the stored iterate (obca_warm_start) */
 
 /* rows kept per instance for the following obca_solve calls; 0 (default) turns recording off.  Takes B * capacity *
  * OBCA_HIST_FIELDS doubles of device memory from the stream-ordered pool, released by obca_destroy or a later call.
@@ -221,6 +226,25 @@ int obca_set_history(ObcaHandle* h, int32_t capacity);
 /* the record of the last obca_solve: rows (B, capacity, OBCA_HIST_FIELDS) dev, may be NULL; count (B) dev int32 = heads
  * evaluated (may exceed capacity), may be NULL.  An error when recording is off. */
 int obca_get_history(ObcaHandle* h, double* rows, int32_t* count, void* stream);
+
+/* ---- warm start from the stored primal-dual iterate (IPOPT: warm_start_init_point = yes) ----------------------------------
+ * Every instance keeps its iterate x, zL, zU (nx each) and y (ny) in device memory, in the internal layout that obca_layout
+ * describes; a solve leaves its final iterate there.  An instance armed by obca_warm_start starts the first interior-point run
+ * of the next obca_solve from that iterate: the user variables of x are kept, the slacks and elastic variables are recomputed
+ * from them, x is pushed into its bounds by warm_start_bound_push, zL / zU are raised to at least warm_start_mult_bound_push
+ * (0 where there is no bound), y is kept, and mu starts at mu0[b] (if given and > 0) or warm_start_mu_init, at least the
+ * smallest mu of the solve.  The solve consumes the arm; restarts inside the solve (dual restoration, raised penalty weight)
+ * start cold.  All calls below are stream ordered, do not synchronise the host and do not allocate (graph capturable). */
+/* dev pointers, any may be NULL: x, zL, zU (B,nx), y (B,ny); mu (B) = barrier parameter at the end of the last solve */
+int obca_get_iterate(ObcaHandle* h, double* x, double* y, double* zL, double* zU, double* mu, void* stream);
+/* dev pointers, any may be NULL (that part of the stored iterate is kept) */
+int obca_set_iterate(ObcaHandle* h, const double* x, const double* y, const double* zL, const double* zU, void* stream);
+/* MPC mode only: every node-indexed entry of the stored x, zL, zU and y of every instance moves one node towards the start of
+ * the horizon, the last valid node is held (VehicleFollower._adv_onestep for the whole iterate); YINIT, YCONT, YTERM, oDT stay */
+int obca_shift_iterate(ObcaHandle* h, void* stream);
+/* arm the next obca_solve: instance b starts warm when mask[b] != 0 (mask NULL: every instance); mask (B) int32 dev;
+ * mu0 (B) dev or NULL (warm_start_mu_init).  The warm_start_* options in force at this call apply. */
+int obca_warm_start(ObcaHandle* h, const int32_t* mask, const double* mu0, void* stream);
 
 /* number of kernels this handle has launched so far (bench.py "gpu_launches") */
 int64_t obca_launch_count(const ObcaHandle* h);
